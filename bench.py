@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- recommend() users/sec of the B200 score + top-K engine on BASELINE.json's configurations.
 
-    python bench.py --gpus N --steps K --warmup W [--config c2|c3|c4|c5] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--config c2|c3|c4|c5] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (score every user against the catalogue, mask viewed items, keep the K best)
 over one batch of synthetic users (SURVEY.md section 8d synthetic inputs: N(0,1)/sqrt(d) factors, fixed seeds, ~100 viewed
@@ -22,6 +22,10 @@ items per user).  Named workloads (BASELINE.json `configs[1..4]`; the default is
            `rectools_b200.install()`, users/sec incl. the host code around the ranker (N = 1, when the package is staged)
   --impl reference : the reference's CPU path (restatement of implicit.cpu.topk: BLAS sgemm + OpenMP select, all host
            threads) on a bounded sample of the same workload, rank 0 only.
+  --dump-outputs DIR : after the timed steps, write what the last timed step returned (top-K ids, scores, counts; rank 0)
+           as DIR/<name>.npy for output-by-output comparison of two builds: `rows` (the users), `ids` and `counts` in
+           float64, `scores` in float32.  Inputs are seeded, so equal arguments give equal inputs; above DUMP_BYTES a
+           fixed, seeded sample of the users is written.
 """
 from __future__ import annotations
 
@@ -37,8 +41,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ of the modules imported below is written there
 
 BLOCK = 65536
+DUMP_BYTES = 64_000_000  # --dump-outputs: the whole dump (all .npy files) stays below this
 
 
 def gen_factors(n, d, seed, lo=0, hi=None):
@@ -67,6 +73,23 @@ def gen_viewed(n_users, n_items, per_user, seed=2):
         cols[r0:r1] = c
     indptr = np.arange(n_users + 1, dtype=np.int64) * per_user
     return indptr, cols.reshape(-1)
+
+
+def dump_outputs(out_dir, rows, ids, scores, counts):
+    """Write the top-K result of `rows` (global user indices) under `out_dir`: every user when it fits DUMP_BYTES, else a
+    seeded sample of users (sorted, the same for every run with the same shapes)."""
+    ids, scores, counts = np.asarray(ids).reshape(len(rows), -1), np.asarray(scores).reshape(len(rows), -1), np.asarray(counts)
+    k = ids.shape[1]
+    per_row = 8 + 8 * k + 4 * k + 8  # rows, ids (float64), scores (float32), counts (float64)
+    n_keep = min(len(rows), (DUMP_BYTES - 4 * 128) // per_row)  # (4 * 128: the .npy headers)
+    sel = np.arange(len(rows))
+    if n_keep < len(rows):
+        sel = np.sort(np.random.default_rng(20260).choice(len(rows), n_keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rows.npy"), np.asarray(rows)[sel].astype(np.float64))
+    np.save(os.path.join(out_dir, "ids.npy"), ids[sel].astype(np.float64))
+    np.save(os.path.join(out_dir, "scores.npy"), scores[sel].astype(np.float32))
+    np.save(os.path.join(out_dir, "counts.npy"), counts[sel].astype(np.float64))
 
 
 class ClockSampler:
@@ -192,10 +215,14 @@ def run_reference(a):
     for s in range(a.warmup + a.steps):
         lo = (s * n_s) % max(1, len(users) - n_s + 1)
         t0 = time.perf_counter()
-        cpu_baseline.topk_cpu(items, users[lo : lo + n_s], a.k, norms, csr[lo : lo + n_s], num_threads=threads)
+        last = cpu_baseline.topk_cpu(items, users[lo : lo + n_s], a.k, norms, csr[lo : lo + n_s], num_threads=threads)
         dt = time.perf_counter() - t0
         if s >= a.warmup:
             times.append(dt)
+    if a.dump_outputs:
+        ids, scores = last
+        # (like implicit's topk, topk_cpu leaves filtered items in the rows with score -FLT_MAX; they are not results)
+        dump_outputs(a.dump_outputs, np.arange(lo, lo + ids.shape[0]), ids, scores, (scores > -np.finfo(np.float32).max).sum(axis=1))
     total = sum(times)
     value = n_s * len(times) / total
     line = {
@@ -299,10 +326,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-model", action="store_true", help="skip the model.recommend() leg")
     ap.add_argument("--no-share", action="store_true", help="N > 1: no threshold sharing between the item shards")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's top-K result as DIR/<name>.npy (see the module docstring)")
     ap.add_argument("--item-shards", type=int, default=0,
                     help="N > 1: item shards I (a divisor of N); the ranks form I item shards x N/I user groups.  0 = N (the north-star "
                          "scheme: every rank ranks all users against 1/N of the catalogue); 1 = plain user sharding")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 0)
     resolve_config(a)
 
@@ -452,6 +483,12 @@ def main():
     sampler.mark()
     total_ms = timed(step_resident, 0, a.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        if world == 1:
+            dump_outputs(a.dump_outputs, np.arange(u0, u1), o_ids.cpu().numpy(), o_sc.cpu().numpy(), o_cnt.cpu().numpy())
+        else:  # rank 0 holds the merged result of the whole job
+            ids = result["ids"].cpu().numpy()
+            dump_outputs(a.dump_outputs, np.arange(ids.shape[0]), ids, result["sc"].cpu().numpy(), result["cnt"].cpu().numpy())
     timed_launches = launches[0]
     timed_stats = list(stats_log)
     value = n_users_all * a.steps / (total_ms / 1e3)  # whole job: all user groups

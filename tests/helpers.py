@@ -223,3 +223,56 @@ class FakeVectorModel:
 
     def recommend_to_items(self, *args, **kwargs):
         raise AssertionError("the vectorised path should not have delegated")
+
+
+def fake_rectools(monkeypatch):
+    """Stand-in modules for the names `rectools_b200.install()` / `make_similarity_module()` rebind or subclass
+    (`rectools.models.{vector,ease}.ImplicitRanker`, `VectorModel` / `ModelBase.recommend{,_to_items}`,
+    `rectools.models.nn.transformers.similarity.DistanceSimilarityModule`), registered in `sys.modules` for one test.
+    Test infrastructure only: the behaviour of the reference behind those names is pinned by tests/golden."""
+    import enum
+    import sys
+    import types
+
+    import torch
+
+    class Distance(enum.Enum):  # rectools/models/rank/rank.py: the values are the contract
+        DOT = "dot"
+        COSINE = "cosine"
+        EUCLIDEAN = "euclidean"
+
+    class ImplicitRanker:  # the stock ranker the two modules import by name
+        pass
+
+    class ModelBase:
+        def recommend(self, *args, **kwargs):
+            raise NotImplementedError
+
+        def recommend_to_items(self, *args, **kwargs):
+            raise NotImplementedError
+
+    class VectorModel(ModelBase):
+        pass
+
+    class DistanceSimilarityModule(torch.nn.Module):
+        def __init__(self, distance="dot"):
+            super().__init__()
+            self.distance = Distance(distance)
+
+        def forward(self, session_embs, item_embs, candidate_item_ids=None):  # any fixed function: inherited or not
+            logits = session_embs @ item_embs.T
+            return logits if candidate_item_ids is None else torch.gather(logits, -1, candidate_item_ids)
+
+    mods = {name: types.ModuleType(name) for name in (
+        "rectools", "rectools.models", "rectools.models.base", "rectools.models.vector", "rectools.models.ease",
+        "rectools.models.nn", "rectools.models.nn.transformers", "rectools.models.nn.transformers.similarity")}
+    mods["rectools.models.base"].ModelBase = ModelBase
+    mods["rectools.models.vector"].__dict__.update(VectorModel=VectorModel, ImplicitRanker=ImplicitRanker, Distance=Distance)
+    mods["rectools.models.ease"].__dict__.update(ImplicitRanker=ImplicitRanker, Distance=Distance)
+    mods["rectools.models.nn.transformers.similarity"].DistanceSimilarityModule = DistanceSimilarityModule
+    for name, mod in mods.items():
+        parent, _, child = name.rpartition(".")
+        if parent:
+            setattr(mods[parent], child, mod)
+        monkeypatch.setitem(sys.modules, name, mod)
+    return types.SimpleNamespace(**mods)

@@ -4,14 +4,18 @@
 like the built `.so`), `oracle/implicit_stub` stands in for the third-party `implicit` (its top-k = the CPU oracle).  Every
 test computes the expectation with the stock reference path (`ImplicitRanker` -> stub top-k on the CPU, `TorchRanker` on the
 CPU) and then the same call after `rectools_b200.install()` / with `make_similarity_module()`: the frames must agree
-(ids exact; near-ties of the fp32 reference arithmetic may swap neighbours within `tie_tol`)."""
+(ids exact; near-ties of the fp32 reference arithmetic may swap neighbours within `tie_tol`).  The similarity-module seam
+compares with the stock module's results stored in tests/golden/similarity_module.npz and runs without the package."""
+import os
+
 import numpy as np
 import pytest
 
 from oracle import stage_reference
-from tests.helpers import assert_same_ranking
+from tests.helpers import GOLDEN, assert_same_ranking, fake_rectools
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not stage_reference.available(), reason="reference package not staged (oracle/_ref)")]
+pytestmark = pytest.mark.gpu
+needs_reference = pytest.mark.skipif(not stage_reference.available(), reason="reference package not staged (oracle/_ref)")
 
 
 @pytest.fixture(scope="module")
@@ -40,6 +44,7 @@ def _factors(n, d, seed):
     return (np.random.default_rng(seed).standard_normal((n, d), dtype=np.float32) / np.sqrt(d)).astype(np.float32)
 
 
+@needs_reference
 @pytest.mark.parametrize("fast_recommend", [True, False])
 def test_puresvd_and_injected_als_recommend_through_the_engine(ref, fast_recommend):
     """`install()` + `PureSVDModel.recommend()` and `ImplicitALSWrapperModel.recommend()` (pre-fitted factors injected as in
@@ -82,6 +87,7 @@ def test_puresvd_and_injected_als_recommend_through_the_engine(ref, fast_recomme
         rectools_b200.uninstall()
 
 
+@needs_reference
 def test_in_place_refit_reaches_the_device(ref):
     """VERDICT r1 weak #3: factors changed IN PLACE between two `recommend()` calls must give fresh results."""
     import rectools_b200
@@ -105,6 +111,7 @@ def test_in_place_refit_reaches_the_device(ref):
     assert not first["item_id"].equals(second["item_id"])
 
 
+@needs_reference
 def test_ease_sparse_subjects_through_install(ref):
     """SURVEY 8 f-4: `EASEModel._recommend_u2i` hands the user x item CSR as SUBJECT factors (ease.py:134-161); the engine
     scores it sparse (SpMM + streaming top-k) instead of densifying users x items."""
@@ -132,21 +139,23 @@ def test_ease_sparse_subjects_through_install(ref):
 
 
 @pytest.mark.parametrize("distance", ["dot", "cosine"])
-def test_transformer_similarity_module_seam(ref, distance):
+def test_transformer_similarity_module_seam(monkeypatch, distance):
     """SURVEY 8 a13 / f-3: `DistanceSimilarityModule._recommend_u2i` (similarity.py:117-140) with `B200TorchRanker` under it
     (`make_similarity_module()`), called the way `TransformerLightningModuleBase._recommend_u2i` does (lightning.py:402-426):
     device-resident `item_embs` with the PAD row first, whitelist = the non-PAD items (nn/transformers/base.py:543-544),
     filter CSR over all token columns.  DOT = SASRec / BERT4Rec, COSINE = HSTU's default (hstu.py:696-703)."""
     import torch
-    from rectools.models.nn.transformers.similarity import DistanceSimilarityModule
     from scipy import sparse
 
     from rectools_b200.integration import make_similarity_module
 
+    DistanceSimilarityModule = fake_rectools(monkeypatch).rectools.models.nn.transformers.similarity.DistanceSimilarityModule
+    gold = np.load(os.path.join(GOLDEN, "similarity_module.npz"))
+
     n_users, n_tokens, d, k = 3000, 20_001, 64, 10  # token 0 = PAD
-    g = torch.Generator().manual_seed(7)
-    user_embs = torch.randn((n_users, d), generator=g) / d**0.5
-    item_embs = torch.randn((n_tokens, d), generator=g) / d**0.5
+    rng = np.random.default_rng(7)  # (numpy: the same values on every host, unlike torch's vectorised CPU sampler)
+    user_embs = torch.from_numpy(rng.standard_normal((n_users, d), dtype=np.float32) / np.float32(d**0.5))
+    item_embs = torch.from_numpy(rng.standard_normal((n_tokens, d), dtype=np.float32) / np.float32(d**0.5))
     item_embs[0] = 0.0
     user_ids = np.random.default_rng(0).permutation(n_users)[:2000]
     rng = np.random.default_rng(1)
@@ -157,8 +166,7 @@ def test_transformer_similarity_module_seam(ref, distance):
     ui.data[:] = 1.0
     whitelist = np.arange(1, n_tokens)
 
-    stock = DistanceSimilarityModule(distance=distance)
-    e_users, e_ids, e_scores = stock._recommend_u2i(user_embs, item_embs, user_ids, k, whitelist, ui)  # pylint: disable=protected-access
+    e_users, e_ids, e_scores = (gold[f"gpu|{distance}|f32|{name}"] for name in ("users", "ids", "scores"))
     ours = make_similarity_module()(distance=distance)
     assert isinstance(ours, DistanceSimilarityModule)
     dev = torch.device("cuda:0")
@@ -169,6 +177,6 @@ def test_transformer_similarity_module_seam(ref, distance):
     # bf16 item embeddings stay 16-bit all the way to the engine (exact widening there): same ids as the fp32 path on the
     # bf16-rounded values
     emb16 = item_embs.to(torch.bfloat16)
-    e2 = stock._recommend_u2i(user_embs, emb16.float(), user_ids, k, whitelist, ui)  # pylint: disable=protected-access
+    e2 = tuple(gold[f"gpu|{distance}|bf16|{name}"] for name in ("users", "ids", "scores"))  # the stock module on emb16.float()
     o2 = ours._recommend_u2i(user_embs, emb16.to(dev), user_ids, k, whitelist, ui)  # pylint: disable=protected-access
     assert_same_ranking(o2[1], o2[2], e2[1], e2[2], rtol=3e-5, atol=3e-6, tie_tol=3e-6)

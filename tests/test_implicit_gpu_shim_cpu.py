@@ -1,18 +1,14 @@
 """CPU: the `implicit.gpu` stand-ins (`rectools_b200/implicit_gpu.py`, the lowest seam of SURVEY section 8b) make the UNMODIFIED
 reference `ImplicitRanker(..., use_gpu=True)` (rank_implicit.py:148-185, :250-262) produce the same triplets as its CPU path.
 The top-k provider behind `KnnQuery.topk` is the oracle here (injected); on a B200 it is the engine (tests/test_gpu_parity.py).
-Needs the reference checkout (build container only; skipped on the GPU box)."""
-import os
-import sys
-
+Runs the reference package itself, so it needs it staged in oracle/_ref (`oracle.stage_reference`); skipped without it."""
 import numpy as np
 import pytest
 from scipy import sparse
 
-REF = "/root/reference"
-STUB = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "oracle", "implicit_stub")
+from oracle import stage_reference
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "rectools")), reason="reference checkout not present")
+pytestmark = pytest.mark.skipif(not stage_reference.available(), reason="reference package neither staged nor checked out")
 
 
 def _oracle_backend(items, queries, k, item_norms, csr):
@@ -24,7 +20,7 @@ def _oracle_backend(items, queries, k, item_norms, csr):
 
 @pytest.fixture()
 def patched():
-    sys.path[:0] = [REF, os.path.abspath(STUB)]
+    added = stage_reference.add_to_path()
     from rectools_b200 import implicit_gpu
 
     implicit_gpu.patch_implicit_gpu(backend=_oracle_backend)
@@ -35,11 +31,7 @@ def patched():
     import implicit.gpu
 
     assert implicit.gpu.HAS_CUDA is False and ri.HAS_CUDA is False
-    for m in [k for k in sys.modules if k.startswith("rectools.") or k == "rectools" or k.startswith("implicit")]:
-        sys.modules.pop(m, None)
-    for p_ in (REF, os.path.abspath(STUB)):
-        if p_ in sys.path:
-            sys.path.remove(p_)
+    stage_reference.remove_from_path(added)
 
 
 @pytest.mark.parametrize("distance", ["DOT", "COSINE", "EUCLIDEAN"])
